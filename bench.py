@@ -642,6 +642,36 @@ def _view(ptr, n, typestr, owner):
     return _View(ptr, max(int(n), 0), typestr, owner)
 
 
+DUMP_ROWS = 1 << 21  # rows of the pipeline's result written by --dump-outputs: 32 MiB of .npy files
+
+
+def dump_pipeline_output(torch, out, n, out_dir, prefix=""):
+    """Writes the float32 column the pipeline returns as .npy files under `out_dir`, so that two builds can be compared
+    output for output: result_values (0.0 where null), result_validity (1.0 / 0.0), result_rows (the row numbers) and
+    result_null_count (of the whole column).  Above DUMP_ROWS rows the column is sampled at one seeded row of each of
+    DUMP_ROWS equal strata, the same rows for every run with the same --rows."""
+    import numpy as np
+    if n <= DUMP_ROWS:
+        rows = np.arange(n, dtype=np.int64)
+    else:
+        stride = n // DUMP_ROWS
+        rows = np.arange(DUMP_ROWS, dtype=np.int64) * stride + np.random.default_rng(SEED).integers(0, stride, DUMP_ROWS)
+    r = torch.from_numpy(rows).to("cuda") + out.offset
+    vals = torch.as_tensor(_view(out.buffers[1].ptr, out.offset + n, "<f4", out), device="cuda")[r]
+    if out.buffers[0] is not None:
+        bits = torch.as_tensor(_view(out.buffers[0].ptr, (out.offset + n + 7) // 8, "|u1", out), device="cuda")
+        valid = ((bits[r >> 3] >> (r & 7).to(torch.uint8)) & 1).bool()
+    else:
+        valid = torch.ones(len(rows), dtype=torch.bool, device="cuda")
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"result_values": torch.where(valid, vals, 0.0).cpu().numpy(),  # a null slot's bytes are unspecified
+              "result_validity": valid.to(torch.float32).cpu().numpy(),
+              "result_rows": rows.astype(np.float64),
+              "result_null_count": np.array([out.null_count], dtype=np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # configs[2] / configs[3] sharded over the ranks (strong scaling, one exchange each)
 # ------------------------------------------------------------------------------------------------
@@ -894,14 +924,18 @@ def run_gpu(args):
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     sync_all()
     start.record(stream)
-    for _ in range(args.steps):
+    for step in range(args.steps):
         out = pipeline(values, indices, other)
-        del out
+        if step < args.steps - 1:  # the last step's result outlives the loop for --dump-outputs
+            del out
     stop.record(stream)
     sync_all()
     total_ms = max_over_ranks(start.elapsed_time(stop))
     launches = lib.b2_launch_count() - launches0
     clocks = sampler.summary() if sampler else None
+    if args.dump_outputs:
+        dump_pipeline_output(torch, out, n, args.dump_outputs, f"rank{rank}_" if world > 1 else "")
+    del out
     ms_per_step = total_ms / args.steps
     value = n * world / (ms_per_step * 1e-3)
 
@@ -1092,7 +1126,13 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the `configs` array (c1/c3/c4/c5 at full size, N = 1 only)")
     ap.add_argument("--no-multi", action="store_true", help="skip the sharded group-by / sort legs")
     ap.add_argument("--unfused", action="store_true", help="run the pipeline as three calls (take, cast, add) instead of the fused kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result column of the last timed step (sampled above 2^21 rows) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm runs in oracle/_ref/ref_bench and returns timings only")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
