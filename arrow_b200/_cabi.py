@@ -131,6 +131,7 @@ PROTOTYPES = [
     ("b2_sort_indices_multi", C.c_int, [_P, _A, C.c_int, C.POINTER(C.c_int32), C.c_int, _A, _P]),
     ("b2_hash_join", C.c_int, [_P, _A, _A, C.c_int, C.c_int, _A, _A, _P]),
     ("b2_select_k", C.c_int, [_P, _A, C.c_int64, C.c_int, C.c_int, _A, _P]),
+    ("b2_sort_strings_path", C.c_int, [_P, _A, C.POINTER(C.c_int32), _P]),
     ("b2_grouper_create", C.c_int, [_P, C.POINTER(C.c_int32), C.c_int, C.POINTER(_P)]),
     ("b2_grouper_destroy", None, [_P]),
     ("b2_grouper_consume", C.c_int, [_P, _A, _A, _P]),

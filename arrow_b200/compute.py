@@ -79,6 +79,15 @@ def _require_numeric(t: pa.DataType) -> None:
         raise pa.ArrowNotImplementedError(f"Function has no kernel matching input types ({t}) on arrow_b200 device arrays")
 
 
+_SORTABLE_STRING_TYPES = (pa.utf8(), pa.large_utf8(), pa.binary(), pa.large_binary())
+
+
+def _require_sortable(t: pa.DataType) -> None:
+    """Sort keys: the numeric types and utf8 / large_utf8 / binary / large_binary (ordered byte-wise, unsigned)."""
+    if t not in _SORTABLE_STRING_TYPES:
+        _require_numeric(t)
+
+
 def _as_scalar(x) -> pa.Scalar:
     if isinstance(x, pa.Scalar):
         return x
@@ -432,6 +441,15 @@ def sort_payload(arr: DeviceArray, payload: DeviceArray, order="ascending", null
     return _out(ctx, cout, pa.uint64())
 
 
+def sort_strings_path(arr: DeviceArray) -> str:
+    """which path the sort of this utf8 / binary column takes: "dict" (sort the distinct values, then their ranks) or
+    "refine" (7-byte prefix rounds) -- B2_SORT_STRINGS_PATH when set, else the sampled estimate (csrc/sort_strings.cu)"""
+    ctx = arr.ctx
+    ca, p = arr._c(), C.c_int32(0)
+    check(ctx.lib.b2_sort_strings_path(ctx.handle, C.byref(ca), C.byref(p), ctx.stream))
+    return "dict" if p.value else "refine"
+
+
 def sort_indices(arr, sort_keys=None, null_placement="at_end", order=None) -> DeviceArray:
     """sort_indices meta function (kernels/vector_sort.cc:850-1027): on one array, or -- given a mapping
     {name: DeviceArray} (a record batch / table of device columns) and sort_keys = [(name, order), ...] -- the
@@ -444,7 +462,7 @@ def sort_indices(arr, sort_keys=None, null_placement="at_end", order=None) -> De
             name, o = (k[0], k[1]) if isinstance(k, (tuple, list)) else (k, "ascending")
             if name not in arr:
                 raise pa.ArrowInvalid(f"No match for FieldRef.Name({name})")
-            _require_numeric(arr[name].type)
+            _require_sortable(arr[name].type)
             cols.append(arr[name])
             orders.append(_order(o))
         ctx = cols[0].ctx
@@ -472,7 +490,7 @@ def select_k_unstable(arr: DeviceArray, k: int, sort_keys=None, null_placement="
         if len(sort_keys) != 1:
             raise pa.ArrowNotImplementedError("arrow_b200 select_k_unstable: one sort key (use sort_indices for several)")
         o = sort_keys[0][1] if isinstance(sort_keys[0], (tuple, list)) else "ascending"
-    _require_numeric(arr.type)
+    _require_sortable(arr.type)
     ctx = arr.ctx
     ca, cout = arr._c(), cabi.B2Array()
     check(ctx.lib.b2_select_k(ctx.handle, C.byref(ca), int(k), _order(o), _placement(null_placement), C.byref(cout), ctx.stream))

@@ -509,7 +509,8 @@ class SortIndicesFunction : public cp::MetaFunction {
         if (chunked->num_chunks() != 1) return Status::NotImplemented("arrow_b200 sort_indices: device tables must hold one chunk per column");
         data = chunked->chunk(0)->data();
       }
-      if (!arrow::is_integer(data->type->id()) && !arrow::is_floating(data->type->id()))
+      const Type::type id = data->type->id();
+      if (!arrow::is_integer(id) && !arrow::is_floating(id) && !arrow::is_base_binary_like(id))
         return Status::NotImplemented("arrow_b200 sort_indices: sort key of type ", data->type->ToString());
       ARROW_RETURN_NOT_OK(DataToB2(*data, &keys[k]));
       orders[k] = so.sort_keys[k].order == cp::SortOrder::Descending ? 1 : 0;
@@ -541,7 +542,7 @@ class SelectKFunction : public cp::MetaFunction {
     if (so.k < 0) return Status::Invalid("select_k_unstable requires a nonnegative `k`, got ", so.k);
     if (so.sort_keys.size() != 1) return Status::Invalid("select_k_unstable on an array takes exactly one sort key");
     const auto& type = *args[0].type();
-    if (!arrow::is_integer(type.id()) && !arrow::is_floating(type.id()))
+    if (!arrow::is_integer(type.id()) && !arrow::is_floating(type.id()) && !arrow::is_base_binary_like(type.id()))
       return Status::NotImplemented("arrow_b200 select_k_unstable: values of type ", type.ToString());
     B2Array v, o;
     ARROW_RETURN_NOT_OK(DataToB2(*args[0].array(), &v));
@@ -632,7 +633,9 @@ static Status AddSelectionFunctions(cp::FunctionRegistry* reg, Runtime* rt) {
 
   auto sort = std::make_shared<Forwarding<cp::VectorFunction>>("array_sort_indices", cp::Arity::Unary(),
                                                                DocFor({"array"}, "ArraySortOptions"), &kSortDefaults);
-  for (const auto& ty : NumericTypes()) {
+  std::vector<std::shared_ptr<arrow::DataType>> sort_types = NumericTypes();
+  for (const auto& ty : arrow::BaseBinaryTypes()) sort_types.push_back(ty);  // utf8, large_utf8, binary, large_binary
+  for (const auto& ty : sort_types) {
     ARROW_RETURN_NOT_OK(sort->AddKernel(MakeVectorKernel(rt, {cp::InputType(ty)}, cp::OutputType(arrow::uint64()), SortExec,
                                                          OptionsState<cp::ArraySortOptions>::Init)));
   }

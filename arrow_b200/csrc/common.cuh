@@ -180,6 +180,18 @@ __device__ __forceinline__ T ld_hint(const T* p, uint64_t pol) {
   return out;
 }
 
+// nbytes (1..8) bytes at p, little-endian, zero-extended; funnel-shifts two aligned 8-byte loads, and only aligned
+// words holding an addressed byte are dereferenced, so it never reads past the word holding a buffer's last byte
+__device__ __forceinline__ uint64_t load_bytes8(const uint8_t* p, int nbytes) {
+  const uintptr_t u = reinterpret_cast<uintptr_t>(p);
+  const uint64_t* a = reinterpret_cast<const uint64_t*>(u & ~uintptr_t(7));
+  const int skip = static_cast<int>(u & 7);
+  uint64_t v = __ldg(a) >> (skip * 8);
+  if (skip && 8 - skip < nbytes) v |= __ldg(a + 1) << (64 - skip * 8);
+  if (nbytes < 8) v &= (1ull << (8 * nbytes)) - 1ull;
+  return v;
+}
+
 __device__ __forceinline__ unsigned lane_id() { return threadIdx.x & 31; }
 __device__ __forceinline__ unsigned lanemask_lt() {
   unsigned m;

@@ -57,17 +57,6 @@ struct Owned {
   }
 };
 
-// nbytes (1..8) bytes at p, zero-extended; only aligned words holding an addressed byte are dereferenced
-__device__ __forceinline__ uint64_t load_bytes8(const uint8_t* p, int nbytes) {
-  const uintptr_t u = reinterpret_cast<uintptr_t>(p);
-  const uint64_t* a = reinterpret_cast<const uint64_t*>(u & ~uintptr_t(7));
-  const int skip = static_cast<int>(u & 7);
-  uint64_t v = __ldg(a) >> (skip * 8);
-  if (skip && 8 - skip < nbytes) v |= __ldg(a + 1) << (64 - skip * 8);
-  if (nbytes < 8) v &= (1ull << (8 * nbytes)) - 1ull;
-  return v;
-}
-
 __device__ __forceinline__ uint64_t mix64(uint64_t h) {
   h ^= h >> 30;
   h *= 0xbf58476d1ce4e5b9ull;

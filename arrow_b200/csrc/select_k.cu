@@ -1,4 +1,4 @@
-// select_k.cu -- select_k_unstable over one numeric column: the indices of the first k rows of the sorted order.
+// select_k.cu -- select_k_unstable over one numeric, utf8 or binary column: the indices of the first k rows of the sorted order.
 //
 // Replaces ArraySelector (kernels/vector_select_k.cc:157-232: null-like partition, then a k-element heap over the
 // non-null values) -- k log k work per row on one CPU thread.  "Unstable" only frees the tie order; this implementation
@@ -16,6 +16,7 @@
 
 #include "common.cuh"
 #include "context.h"
+#include "sort_internal.h"
 
 using namespace b2;
 
@@ -44,6 +45,48 @@ int full_sort_prefix(B2Context* ctx, const B2Array* values, int64_t k, int order
   if (k < out->length) out->length = k;  // a prefix view of the same buffer
   return B2_OK;
 }
+
+// utf8 / binary: the round-0 keys of the string sort (sort_strings.cu) order the rows wherever two keys differ, so the
+// numeric selection over the key column gives a threshold key T (the last key it selected); every row that can be among
+// the first k has a key at or before T, ties included.  Those candidates are sorted as strings.
+int select_k_strings(B2Context* ctx, const B2Array* values, int64_t k, int order, int null_placement, B2Array* out,
+                     void* stream) {
+  const int64_t n = values->length;
+  cudaStream_t s = ctx->pick(stream);
+  const bool maybe_nulls = values->null_count != 0 && values->validity;
+  if (n < (1 << 20) || k * 8 > n || (null_placement == 0 && maybe_nulls))
+    return full_sort_prefix(ctx, values, k, order, null_placement, out, stream);
+  Out keys(ctx, s), sel(ctx, s), pick(ctx, s);
+  B2_RETURN_NOT_OK(string_prefix_keys(ctx, values, &keys.a, s));
+  B2_RETURN_NOT_OK(b2_select_k(ctx, &keys.a, k, order, null_placement, &sel.a, stream));
+  B2Array last = sel.a;
+  last.offset += k - 1;
+  last.length = 1;
+  B2_RETURN_NOT_OK(b2_take(ctx, &keys.a, &last, 0, &pick.a, stream));
+  if (pick.a.null_count != 0) return full_sort_prefix(ctx, values, k, order, null_placement, out, stream);  // < k valid rows
+  uint64_t bits = 0;
+  B2_CUDA(cudaMemcpyAsync(&bits, pick.a.data, sizeof(bits), cudaMemcpyDeviceToHost, s));
+  B2_CUDA(cudaStreamSynchronize(s));
+
+  B2Scalar t{bits, B2_UINT64, 1};
+  B2Value l{&keys.a, nullptr}, r{nullptr, &t};
+  Out mask(ctx, s), cand_rows(ctx, s);
+  B2_RETURN_NOT_OK(b2_compare(ctx, order == 0 ? B2_LESS_EQUAL : B2_GREATER_EQUAL, &l, &r, &mask.a, stream));
+  B2_RETURN_NOT_OK(b2_filter_indices(ctx, &mask.a, /*DROP=*/0, &cand_rows.a, stream));
+  const int64_t m = cand_rows.a.length;
+  if (m < k || m * 2 > n) return full_sort_prefix(ctx, values, k, order, null_placement, out, stream);
+
+  Out cand(ctx, s), perm(ctx, s), picked(ctx, s), wide(ctx, s);
+  B2_RETURN_NOT_OK(b2_take(ctx, values, &cand_rows.a, 0, &cand.a, stream));
+  B2_RETURN_NOT_OK(b2_sort_indices(ctx, &cand.a, order, null_placement, &perm.a, stream));
+  B2Array first_k = perm.a;
+  first_k.length = k;
+  B2_RETURN_NOT_OK(b2_take(ctx, &cand_rows.a, &first_k, 0, &picked.a, stream));
+  B2CastOptions to_u64{B2_UINT64, 1, 1, 0};
+  B2_RETURN_NOT_OK(b2_cast_numeric(ctx, &picked.a, &to_u64, &wide.a, stream));
+  wide.give(out);
+  return B2_OK;
+}
 }  // namespace
 
 extern "C" int b2_select_k(B2Context* ctx, const B2Array* values, int64_t k, int order, int null_placement, B2Array* out,
@@ -52,7 +95,8 @@ extern "C" int b2_select_k(B2Context* ctx, const B2Array* values, int64_t k, int
   if (k < 0) return set_error(B2_INVALID, "select_k_unstable requires a nonnegative `k`, got %lld", (long long)k);  // vector_select_k.cc:640
   if (order != 0 && order != 1) return set_error(B2_INVALID, "bad sort order %d", order);
   if (null_placement != 0 && null_placement != 1) return set_error(B2_INVALID, "bad null placement %d", null_placement);
-  if (!type_is_numeric(values->type)) return set_error(B2_NOT_IMPLEMENTED, "select_k_unstable: unsupported type id %d", values->type);
+  if (!type_is_numeric(values->type) && !type_is_binary_like(values->type))
+    return set_error(B2_NOT_IMPLEMENTED, "select_k_unstable: unsupported type id %d", values->type);
   const int64_t n = values->length;
   if (k > n) k = n;
   cudaStream_t s = ctx->pick(stream);
@@ -61,6 +105,7 @@ extern "C" int b2_select_k(B2Context* ctx, const B2Array* values, int64_t k, int
     fill_out(out, B2_UINT64, 0, 0, nullptr, nullptr);
     return B2_OK;
   }
+  if (type_is_binary_like(values->type)) return select_k_strings(ctx, values, k, order, null_placement, out, stream);
   const bool is_float = values->type == B2_FLOAT || values->type == B2_DOUBLE;
   // the threshold path only ever selects non-null, non-NaN rows: with nulls (or possibly NaNs) FIRST they would be skipped
   const bool maybe_nulls = values->null_count != 0 && values->validity;

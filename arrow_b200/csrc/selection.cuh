@@ -32,6 +32,26 @@ struct FilterBitmaps {
   }
 };
 
+// warp 0 of a compaction tile: the tile's 64 selection words and, per word, the selected rows before it in the tile
+// (the rank of row r is s_prefix[r >> 6] + popcount of the bits below r in s_sel[r >> 6])
+__device__ __forceinline__ void load_tile_prefix(const BitmapReader& sel, int64_t tile, uint64_t* s_sel, uint32_t* s_prefix) {
+  const unsigned lane = lane_id();
+  const int64_t w0 = tile * kTileWords + 2 * lane;
+  const uint64_t s0 = sel.word(w0), s1 = sel.word(w0 + 1);
+  const int c0 = __popcll(s0), c1 = __popcll(s1);
+  int incl = c0 + c1;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    int v = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += v;
+  }
+  const int excl = incl - c0 - c1;
+  s_sel[2 * lane] = s0;
+  s_sel[2 * lane + 1] = s1;
+  s_prefix[2 * lane] = excl;
+  s_prefix[2 * lane + 1] = excl + c0;
+}
+
 inline int64_t tiles_for(int64_t n) { return (n + kTileRows - 1) / kTileRows; }
 
 // passes 1+2: per-tile exclusive output offsets (int64[n_tiles+1], device), the output

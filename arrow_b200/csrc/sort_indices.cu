@@ -34,6 +34,7 @@
 #include <type_traits>
 
 #include "selection.cuh"
+#include "sort_internal.h"
 
 namespace b2 {
 
@@ -98,23 +99,7 @@ __global__ void __launch_bounds__(kBlock) sort_prepare_kernel(PrepareArgs<T> a) 
   __shared__ uint32_t s_prefix[kTileWords];
   const int64_t tile = blockIdx.x;
   const int64_t row0 = tile * kTileRows;
-  const unsigned lane = lane_id();
-  if (threadIdx.x < 32) {
-    int64_t w0 = tile * kTileWords + 2 * lane;
-    uint64_t s0 = a.valid.word(w0), s1 = a.valid.word(w0 + 1);
-    int c0 = __popcll(s0), c1 = __popcll(s1);
-    int incl = c0 + c1;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      int v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += v;
-    }
-    int excl = incl - c0 - c1;
-    s_sel[2 * lane] = s0;
-    s_sel[2 * lane + 1] = s1;
-    s_prefix[2 * lane] = excl;
-    s_prefix[2 * lane + 1] = excl + c0;
-  }
+  if (threadIdx.x < 32) load_tile_prefix(a.valid, tile, s_sel, s_prefix);
   __syncthreads();
   const int64_t vbase = a.tile_offsets[tile];
   const int64_t nbase = row0 - vbase;  // nulls before this tile
@@ -395,8 +380,20 @@ static int sort_typed(B2Context* ctx, const B2Array* values, int order, int null
   }
   if (nv == 0) return B2_OK;
 
-  // 2. histograms of all digits
-  const int passes = sizeof(T);
+  // 2. the radix passes; the last one writes the uint64 result
+  K* unused_keys;
+  uint32_t* unused_idx;
+  return radix_sort_pairs<K>(ctx, sizeof(T), keysA.as<K>(), idxA.as<uint32_t>(), &keysB, &idxB, (uint32_t)nv, out_values,
+                             &unused_keys, &unused_idx, s);
+}
+
+template <typename K>
+int radix_sort_pairs(B2Context* ctx, int passes, K* keys_a, uint32_t* idx_a, Temp* keys_b, Temp* idx_b, uint32_t n,
+                     uint64_t* final_out, K** keys_out, uint32_t** idx_out, cudaStream_t s) {
+  *keys_out = keys_a;
+  *idx_out = idx_a;
+  if (n == 0) return B2_OK;
+  // histograms of all digits
   Temp hist(ctx, s), dbase(ctx, s);
   B2_RETURN_NOT_OK(hist.alloc(sizeof(unsigned long long) * 8 * kRadix));
   B2_RETURN_NOT_OK(dbase.alloc(sizeof(uint32_t) * 8 * kRadix));
@@ -404,12 +401,10 @@ static int sort_typed(B2Context* ctx, const B2Array* values, int order, int null
   ScalarSlot slot(ctx);
   B2_RETURN_NOT_OK(slot.zero(s));
   {
-    int grid = grid_for(nv, kSortThreads * 16, kSMs * 8);
-    radix_hist_kernel<K><<<grid, kSortThreads, 0, s>>>(keysA.as<K>(), (uint32_t)nv, passes,
-                                                       hist.as<unsigned long long>());
+    int grid = grid_for(n, kSortThreads * 16, kSMs * 8);
+    radix_hist_kernel<K><<<grid, kSortThreads, 0, s>>>(keys_a, n, passes, hist.as<unsigned long long>());
     B2_LAUNCHED();
-    radix_scan_kernel<<<passes, kRadix, 0, s>>>(hist.as<unsigned long long>(), (uint32_t)nv,
-                                                dbase.as<uint32_t>(), slot.dev());
+    radix_scan_kernel<<<passes, kRadix, 0, s>>>(hist.as<unsigned long long>(), n, dbase.as<uint32_t>(), slot.dev());
     B2_LAUNCHED();
   }
   B2_RETURN_NOT_OK(slot.fetch(s));
@@ -418,17 +413,19 @@ static int sort_typed(B2Context* ctx, const B2Array* values, int order, int null
     if (!slot.host()[p]) todo[n_todo++] = p;
 
   if (n_todo == 0) {
-    widen_idx_kernel<<<grid_for(nv, kBlock * 4, kSMs * 8), kBlock, 0, s>>>(idxA.as<uint32_t>(), out_values, nv);
-    B2_LAUNCHED();
+    if (final_out) {
+      widen_idx_kernel<<<grid_for(n, kBlock * 4, kSMs * 8), kBlock, 0, s>>>(idx_a, final_out, n);
+      B2_LAUNCHED();
+    }
     return B2_OK;
   }
-  if (n_todo > 1) {
-    B2_RETURN_NOT_OK(keysB.alloc(sizeof(K) * (size_t)nv));
-    B2_RETURN_NOT_OK(idxB.alloc(sizeof(uint32_t) * (size_t)nv));
+  if (n_todo > 1 || !final_out) {
+    if (!keys_b->ptr) B2_RETURN_NOT_OK(keys_b->alloc(sizeof(K) * (size_t)n));
+    if (!idx_b->ptr) B2_RETURN_NOT_OK(idx_b->alloc(sizeof(uint32_t) * (size_t)n));
   }
-  const uint32_t n_tiles = (uint32_t)((nv + kSortTile - 1) / kSortTile);
+  const uint32_t n_tiles = (uint32_t)((n + kSortTile - 1) / kSortTile);
   Temp lookback(ctx, s);
-  const bool wide = nv >= (1ll << 30);
+  const bool wide = n >= (1u << 30);
   const size_t cell = wide ? sizeof(unsigned long long) : sizeof(uint32_t);
   const size_t lb_bytes = (size_t)n_tiles * kRadix * cell + 256;
   B2_RETURN_NOT_OK(lookback.alloc(lb_bytes));
@@ -439,21 +436,21 @@ static int sort_typed(B2Context* ctx, const B2Array* values, int order, int null
   B2_CUDA(cudaFuncSetAttribute(onesweep_kernel<K, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   B2_CUDA(cudaFuncSetAttribute(onesweep_kernel<K, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   B2_CUDA(cudaFuncSetAttribute(onesweep_kernel<K, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  K* kin = keysA.as<K>();
-  K* kout = keysB.as<K>();
-  uint32_t* iin = idxA.as<uint32_t>();
-  uint32_t* iout = idxB.as<uint32_t>();
+  K* kin = keys_a;
+  K* kout = keys_b->as<K>();
+  uint32_t* iin = idx_a;
+  uint32_t* iout = idx_b->as<uint32_t>();
   for (int t = 0; t < n_todo; ++t) {
     const int p = todo[t];
-    const bool last = t == n_todo - 1;
+    const bool last = final_out && t == n_todo - 1;
     B2_CUDA(cudaMemsetAsync(lookback.ptr, 0, lb_bytes, s));
     OnesweepArgs<K> a;
     a.keys_in = kin;
     a.idx_in = iin;
     a.keys_out = kout;
     a.idx_out = iout;
-    a.final_out = out_values;
-    a.n = (uint32_t)nv;
+    a.final_out = final_out;
+    a.n = n;
     a.shift = p * kRadixBits;
     a.digit_base = dbase.as<uint32_t>() + p * kRadix;
     a.lookback = lookback.ptr;
@@ -469,8 +466,15 @@ static int sort_typed(B2Context* ctx, const B2Array* values, int order, int null
     K* tk = kin; kin = kout; kout = tk;
     uint32_t* ti = iin; iin = iout; iout = ti;
   }
+  *keys_out = kin;
+  *idx_out = iin;
   return B2_OK;
 }
+
+template int radix_sort_pairs<uint32_t>(B2Context*, int, uint32_t*, uint32_t*, Temp*, Temp*, uint32_t, uint64_t*,
+                                        uint32_t**, uint32_t**, cudaStream_t);
+template int radix_sort_pairs<uint64_t>(B2Context*, int, uint64_t*, uint32_t*, Temp*, Temp*, uint32_t, uint64_t*,
+                                        uint64_t**, uint32_t**, cudaStream_t);
 
 }  // namespace b2
 
@@ -496,7 +500,7 @@ static int sort_run(B2Context* ctx, const B2Array* values, int order, int null_p
   if (order != 0 && order != 1) return set_error(B2_INVALID, "bad sort order %d", order);
   if (null_placement != 0 && null_placement != 1) return set_error(B2_INVALID, "bad null placement %d", null_placement);
   if (values->length < 0 || values->offset < 0) return set_error(B2_INVALID, "negative length/offset");
-  if (!type_is_numeric(values->type))
+  if (!type_is_numeric(values->type) && !type_is_binary_like(values->type))
     return set_error(B2_NOT_IMPLEMENTED, "sort_indices: unsupported type id %d", values->type);
   const int64_t n = values->length;
   if (n >= (1ll << 32) - 8192)  // row numbers travel as uint32 between the passes
@@ -505,25 +509,31 @@ static int sort_run(B2Context* ctx, const B2Array* values, int order, int null_p
   B2_CUDA(cudaSetDevice(ctx->device));
   Temp data(ctx, s);
   B2_RETURN_NOT_OK(data.alloc(sizeof(uint64_t) * (size_t)n));
-  if (n > 0) {
-    int st;
-    uint64_t* o = data.as<uint64_t>();
-    switch (values->type) {
-      case B2_INT8: st = sort_typed<int8_t>(ctx, values, order, null_placement, o, s, payload); break;
-      case B2_UINT8: st = sort_typed<uint8_t>(ctx, values, order, null_placement, o, s, payload); break;
-      case B2_INT16: st = sort_typed<int16_t>(ctx, values, order, null_placement, o, s, payload); break;
-      case B2_UINT16: st = sort_typed<uint16_t>(ctx, values, order, null_placement, o, s, payload); break;
-      case B2_INT32: st = sort_typed<int32_t>(ctx, values, order, null_placement, o, s, payload); break;
-      case B2_UINT32: st = sort_typed<uint32_t>(ctx, values, order, null_placement, o, s, payload); break;
-      case B2_INT64: st = sort_typed<int64_t>(ctx, values, order, null_placement, o, s, payload); break;
-      case B2_UINT64: st = sort_typed<uint64_t>(ctx, values, order, null_placement, o, s, payload); break;
-      case B2_FLOAT: st = sort_typed<float>(ctx, values, order, null_placement, o, s, payload); break;
-      default: st = sort_typed<double>(ctx, values, order, null_placement, o, s, payload); break;
-    }
-    if (st != B2_OK) return st;
-  }
+  B2_RETURN_NOT_OK(sort_into(ctx, values, order, null_placement, payload, data.as<uint64_t>(), s));
   fill_out(out, B2_UINT64, n, 0, nullptr, data.release());
   return B2_OK;
+}
+
+int b2::sort_into(B2Context* ctx, const B2Array* values, int order, int null_placement, const uint32_t* payload, uint64_t* o,
+                  cudaStream_t s) {
+  if (values->length == 0) return B2_OK;
+  int st;
+  switch (values->type) {
+    case B2_INT8: st = sort_typed<int8_t>(ctx, values, order, null_placement, o, s, payload); break;
+    case B2_UINT8: st = sort_typed<uint8_t>(ctx, values, order, null_placement, o, s, payload); break;
+    case B2_INT16: st = sort_typed<int16_t>(ctx, values, order, null_placement, o, s, payload); break;
+    case B2_UINT16: st = sort_typed<uint16_t>(ctx, values, order, null_placement, o, s, payload); break;
+    case B2_INT32: st = sort_typed<int32_t>(ctx, values, order, null_placement, o, s, payload); break;
+    case B2_UINT32: st = sort_typed<uint32_t>(ctx, values, order, null_placement, o, s, payload); break;
+    case B2_INT64: st = sort_typed<int64_t>(ctx, values, order, null_placement, o, s, payload); break;
+    case B2_UINT64: st = sort_typed<uint64_t>(ctx, values, order, null_placement, o, s, payload); break;
+    case B2_FLOAT: st = sort_typed<float>(ctx, values, order, null_placement, o, s, payload); break;
+    case B2_STRING: case B2_BINARY: case B2_LARGE_STRING: case B2_LARGE_BINARY:
+      st = sort_strings(ctx, values, order, null_placement, o, s, payload);
+      break;
+    default: st = sort_typed<double>(ctx, values, order, null_placement, o, s, payload); break;
+  }
+  return st;
 }
 
 // Multi-key sort (SortIndices over a record batch / table, kernels/vector_sort.cc:386-600 MultipleKeyRecordBatchSorter
@@ -533,25 +543,6 @@ static int sort_run(B2Context* ctx, const B2Array* values, int order, int null_p
 // B200 design: least-significant key first, every round a STABLE single-key radix sort whose payload is the
 // permutation so far -- round k gathers key k through the current permutation (b2_take) and sorts it with the
 // permutation riding along the radix passes (sort_run's payload), so no comparator and no per-row key tuple exist.
-namespace {
-struct PoolArray {  // a C-ABI output whose buffers go back to the pool unless released
-  B2Context* ctx;
-  cudaStream_t s;
-  B2Array a{};
-  bool owned = false;
-  PoolArray(B2Context* c, cudaStream_t st) : ctx(c), s(st) {}
-  ~PoolArray() { reset(); }
-  void reset() {
-    if (!owned) return;
-    if (a.validity) ctx->free(const_cast<void*>(a.validity), s);
-    if (a.data) ctx->free(const_cast<void*>(a.data), s);
-    if (a.data2) ctx->free(const_cast<void*>(a.data2), s);
-    owned = false;
-    a = B2Array{};
-  }
-};
-}  // namespace
-
 extern "C" int b2_sort_indices_multi(B2Context* ctx, const B2Array* keys, int n_keys, const int32_t* orders, int null_placement,
                                      B2Array* out, void* stream) {
   if (!ctx || !keys || !orders || !out) return set_error(B2_INVALID, "b2_sort_indices_multi: null argument");

@@ -5,6 +5,10 @@
   c3u group-by / dictionary_encode with a large_utf8 key   500M strings from 1M distinct words (not in the default --only list)
   join inner hash join: n/2 probe rows against 10M unique build keys (not in the default --only list)
   c4  SortIndices int64 + validity        1B rows (wide range) and narrow range [0, 4095]
+  sort_utf8         SortIndices large_utf8, n/2 strings from 1M distinct words of 8-16 B (dictionary path)
+  sort_utf8_unique  SortIndices large_utf8, n/5 random strings of 8-32 B (prefix refinement)
+  sort_utf8_prefix  SortIndices large_utf8, n/10 strings sharing a 40-byte prefix (refinement, 7+ rounds)
+                    (the three sort_utf8 configs are not in the default --only list)
   f1  dictionary_encode / value_counts of an int64 column (1M distinct values), 500M rows
   c5  large_utf8 Filter                   500M strings, 0-32 B, null_p 0.1, s = 0.5  (+ dictionary Take)
   cmp compare int64 -> bool               1B rows
@@ -62,6 +66,40 @@ def report(name, n, ms, alg_bytes, extra=None):
     print(json.dumps(line), flush=True)
 
 
+def card():
+    """the GPU the numbers were measured on and its power limit (read only)"""
+    import subprocess
+    q = subprocess.run(["nvidia-smi", "-i", str(torch.cuda.current_device()), "--query-gpu=name,power.limit", "--format=csv,noheader,nounits"],
+                       capture_output=True, text=True).stdout.strip().split(", ")
+    return {"gpu": q[0] if q and q[0] else torch.cuda.get_device_name(), "power_limit_w": float(q[1]) if len(q) > 1 else None}
+
+
+def sort_parity(ctx, out, m, offs, data, gen):
+    """the sort result is a permutation (scatter-count on the device) and 1M seeded sampled adjacent output pairs are in
+    order on the host, equal neighbours in increasing row order"""
+    idx = torch.as_tensor(_cai(out.buffers[1].ptr, m, "<u8"), device="cuda").to(torch.int64)
+    seen = torch.zeros(m, dtype=torch.int32, device="cuda")
+    seen.index_add_(0, idx, torch.ones(m, dtype=torch.int32, device="cuda"))
+    ok = bool((seen == 1).all().item())
+    del seen
+    j = torch.randint(0, m - 1, (1 << 20,), device="cuda", generator=gen)
+    a, b = idx[j], idx[j + 1]
+    del idx
+    host = {}
+    for name, rows in (("a", a), ("b", b)):
+        lo, hi = offs[rows], offs[rows + 1]
+        width = int((hi - lo).max().item())
+        pos = lo.unsqueeze(1) + torch.arange(width, device="cuda")
+        mat = torch.where(pos < hi.unsqueeze(1), data[pos.clamp(max=data.numel() - 1)], torch.zeros((), dtype=torch.uint8, device="cuda"))
+        host[name] = (mat.cpu().numpy(), (hi - lo).cpu().numpy(), rows.cpu().numpy())
+    (ma, la, ra), (mb, lb, rb) = host["a"], host["b"]
+    for i in range(len(ra)):
+        x, y = ma[i, :la[i]].tobytes(), mb[i, :lb[i]].tobytes()
+        if not (x < y or (x == y and ra[i] < rb[i])):
+            return False
+    return ok
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rows", type=int, default=1_000_000_000)
@@ -69,6 +107,9 @@ def main():
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--fused-only", action="store_true", help="c3: stop after the fused group-by")
     ap.add_argument("--groups", type=int, default=0, help="c3: number of distinct keys (default 10M at >= 100M rows)")
+    ap.add_argument("--vocab", default="", help="sort_utf8: comma-separated numbers of distinct words (default 1M at >= 10M strings)")
+    ap.add_argument("--string-paths", default="auto",
+                    help="sort_utf8*: comma-separated sort paths to time on the same column: auto, dict, refine")
     args = ap.parse_args()
     only = set(args.only.split(","))
     n = args.rows
@@ -187,6 +228,50 @@ def main():
             report(f"c4 sort_indices int64 {name}", m, ms, m * 16.125)
             del keys, keys_t, kvalid_t
             ctx.trim()
+
+    sort_utf8 = [(c, None) for c in ("sort_utf8_unique", "sort_utf8_prefix") if c in only]
+    if "sort_utf8" in only:
+        m = n // 2
+        vocabs = [int(v) for v in args.vocab.split(",") if v] or [1_000_000 if m >= 10_000_000 else max(100, m // 100)]
+        sort_utf8 = [("sort_utf8", v) for v in vocabs] + sort_utf8
+    for cfg, vocab in sort_utf8:
+        if cfg == "sort_utf8":  # the c3u column: distinct words of 8-16 B
+            from bench import make_word_column
+            m = n // 2
+            _, offs, data, total = make_word_column(torch, gen, m, vocab)
+            label = f"sort_utf8 sort_indices large_utf8 ({vocab} distinct words of 8-16 B)"
+        else:
+            m = n // 5 if cfg == "sort_utf8_unique" else n // 10
+            prefix = 0 if cfg == "sort_utf8_unique" else 40
+            lens = torch.randint(8, 33, (m,), dtype=torch.int64, device="cuda", generator=gen) + prefix
+            offs = torch.zeros(m + 1, dtype=torch.int64, device="cuda")
+            torch.cumsum(lens, 0, out=offs[1:])
+            total = int(offs[-1].item())
+            data = torch.randint(97, 123, (total + 64,), dtype=torch.uint8, device="cuda", generator=gen)
+            if prefix:
+                starts = offs[:-1]
+                for k in range(prefix):
+                    data[starts + k] = 120  # 'x'
+            del lens
+            label = ("sort_utf8_unique sort_indices large_utf8 (random 8-32 B)" if not prefix else
+                     "sort_utf8_prefix sort_indices large_utf8 (40-byte common prefix + 8-32 random B)")
+        strs = DeviceArray.from_pointers(ctx, pa.large_string(), m, offs.data_ptr(), data2_ptr=data.data_ptr())
+        L = total / m
+        for p in args.string_paths.split(","):
+            if p == "auto":
+                os.environ.pop("B2_SORT_STRINGS_PATH", None)
+            else:
+                os.environ["B2_SORT_STRINGS_PATH"] = p
+            ms = timed(stream, lambda: bc.array_sort_indices(strs), max(1, args.reps - 1), warmup=1)
+            out = bc.array_sort_indices(strs)
+            ok = sort_parity(ctx, out, m, offs, data, gen)
+            # algorithmic bytes: offsets + characters read once, the uint64 permutation written once
+            report(label, m, ms, m * (8 + L + 8), {"mean_len": L, "parity_checksum_ok": ok, "path": bc.sort_strings_path(strs),
+                                                   "path_forced": p != "auto", **card()})
+            del out
+        os.environ.pop("B2_SORT_STRINGS_PATH", None)
+        del strs, offs, data
+        ctx.trim()
 
     if "c5" in only:
         m = n // 2

@@ -299,10 +299,15 @@ B2_API int b2_binary_data_size(B2Context* ctx, const B2Array* array, int64_t* ou
  * PartitionNullsAndNans (kernels/vector_sort_internal.h:113-305).
  * order: 0 = Ascending, 1 = Descending; null_placement: 0 = AtStart, 1 = AtEnd
  * (compute/ordering.h:30-44).  out: B2_UINT64, length = values.length, no nulls.
+ * values: a numeric column, or a B2_STRING / B2_BINARY / B2_LARGE_STRING / B2_LARGE_BINARY column ordered
+ * unsigned byte-wise with a proper prefix first (ArrayCompareSorter over base-binary types,
+ * kernels/vector_array_sort.cc:144-178,588-594; csrc/sort_strings.cu).  Fewer than 2^32 - 8192 rows;
+ * character data of any size.  fixed_size_binary, string_view, dictionary and nested values are
+ * B2_NOT_IMPLEMENTED.
  * ------------------------------------------------------------------------- */
 B2_API int b2_sort_indices(B2Context* ctx, const B2Array* values, int order,
                            int null_placement, B2Array* out, void* stream);
-/* The same stable sort, but row i carries payload[i] (B2_UINT32, no nulls) instead of its row number i:
+/* The same stable sort (same value types), but row i carries payload[i] (B2_UINT32, no nulls) instead of its row number i:
  * out[k] = payload of the k-th row in sorted order (B2_UINT64).  The owner GPU of the distributed SortIndices sorts the
  * received (key, global row) pairs with it, so the row numbers ride along the radix passes instead of being gathered
  * afterwards (b2_sort_indices + b2_take = a second, random-access-bound pass). */
@@ -310,13 +315,21 @@ B2_API int b2_sort_payload(B2Context* ctx, const B2Array* values, const B2Array*
                            int null_placement, B2Array* out, void* stream);
 /* Multi-key SortIndices (record batch / table sort, kernels/vector_sort.cc:386-600,850-1027): rows ordered by keys[0],
  * ties by keys[1], ...; orders[k] = 0 ascending / 1 descending per key; one null placement (0 = AtStart, 1 = AtEnd); stable.  Every key column
- * is numeric and of the same length (< 2^32 - 8192 rows).  out: B2_UINT64 row indices. */
+ * is numeric or utf8 / binary (as b2_sort_indices; MultipleKeyRecordBatchSorter over base-binary columns,
+ * kernels/vector_sort.cc:386-600) and of the same length (< 2^32 - 8192 rows).  out: B2_UINT64 row indices. */
 B2_API int b2_sort_indices_multi(B2Context* ctx, const B2Array* keys, int n_keys, const int32_t* orders,
                                  int null_placement, B2Array* out, void* stream);
 
-/* select_k_unstable over one numeric column (ArraySelector, kernels/vector_select_k.cc:157-232): out = the B2_UINT64
- * indices of the first min(k, length) rows in sort order = b2_sort_indices(...)[0:k] (ties in row order).  For k << n the
- * column is read once: a sampled threshold, one compare pass, a sort of the few candidates (csrc/select_k.cu). */
+/* The path b2_sort_indices / b2_sort_payload take for this utf8 / binary column: *out_path = 0 prefix refinement,
+ * 1 dictionary (csrc/sort_strings.cu).  The environment variable B2_SORT_STRINGS_PATH=dict|refine forces a path;
+ * otherwise a strided sample estimates the column's rows per distinct value.  Benchmarks label their measurements with
+ * it and tests pin the selection. */
+B2_API int b2_sort_strings_path(B2Context* ctx, const B2Array* values, int32_t* out_path, void* stream);
+
+/* select_k_unstable over one numeric or utf8 / binary column (ArraySelector, kernels/vector_select_k.cc:157-232, and
+ * its base-binary instantiations): out = the B2_UINT64 indices of the first min(k, length) rows in sort order =
+ * b2_sort_indices(...)[0:k] (ties in row order).  For k << n the column is read once: a sampled threshold, one compare
+ * pass, a sort of the few candidates (csrc/select_k.cu); strings are thresholded on their first 7 bytes. */
 B2_API int b2_select_k(B2Context* ctx, const B2Array* values, int64_t k, int order, int null_placement,
                        B2Array* out, void* stream);
 
